@@ -2,7 +2,7 @@
 """Benchmark of the MLD sampling path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--config headline|1prompt|action512|novae1024] [--scaling weak|strong]
+                    [--config headline|1prompt|action512|novae1024] [--scaling weak|strong] [--dump-outputs DIR]
 
 Default (`--config headline`, the driver's line): motions/sec @ 50-step DDIM text-to-motion, batch 256
 (BASELINE.json configs[2]: 77-token CLIP context, latent 1x256, decode to 196x263, joints).  One "step" = one
@@ -13,6 +13,8 @@ for their own workload; `--scaling strong` shards a fixed total batch instead of
 ``--impl reference`` times the CPU restatement of the reference path (the oracle, pinned against the
 reference's own modules; the reference itself is Python and does not exist on the GPU box) on a bounded sample
 of the same workload.
+``--dump-outputs DIR`` writes what the timed path returned in its last step as ``DIR/<name>.npy`` (float32), so
+that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -27,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree, which may be read-only
 
 _T0 = time.time()
 
@@ -55,6 +58,26 @@ WORKLOADS = {
         total_fixed=False, flop_per_motion=20.18e12, cpu_sample=1,
         workload="no-VAE raw-motion diffusion (trans_dec d=512) B=128/GPU (1024 over 8), 196x263, 1000 DDPM steps, CFG 7.5"),
 }
+
+
+# what the timed path returns per workload (--dump-outputs file name)
+OUTPUT_NAME = {"headline": "joints", "1prompt": "joints", "action512": "feats", "novae1024": "motion"}
+DUMP_LIMIT = 64_000_000      # bytes per dump; a larger output is sampled along its batch dimension
+
+
+def dump_output(path: str, name: str, out, batch_dim: int):
+    """``out`` as float32 ``path/<name>.npy``.  When it exceeds DUMP_LIMIT, a fixed seeded sample of motions
+    along ``batch_dim`` (the same rows for the same shape in every run)."""
+    import numpy as np
+    import torch
+    n = out.shape[batch_dim]
+    keep = min(n, (DUMP_LIMIT - 4096) // (out.numel() // n * 4))          # 4 KB for the .npy header
+    if keep < n:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out = out.index_select(batch_dim, rows.to(out.device))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, f"{name}.npy"), out.float().cpu().numpy())
+    _log(f"dumped {name} {list(out.shape)} ({keep} of {n} motions) to {path}")
 
 
 def _cpu_threads() -> int:
@@ -286,7 +309,12 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the b200 path's result; the reference arm times a sample of the workload")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3) if args.config != "novae1024" else max(args.warmup, 1)
@@ -353,7 +381,7 @@ def main():
             out = eng.sample(cond_d, noise_d, len_list, want=("feats",))["feats"]
             return eng.allgather(out, feats_all) if world > 1 else out
         if world == 1:
-            return eng.sample(cond_d, noise_d, len_list, want=("joints",))
+            return eng.sample(cond_d, noise_d, len_list, want=("joints",))["joints"]
         # the one collective of the path, through the C ABI, on a side stream: batch i's gather overlaps batch i+1
         flip[0] ^= 1
         return eng.sample_gather(cond_d, noise_d, len_list, T=T, out=gathered[flip[0]], wait=False)
@@ -387,7 +415,7 @@ def main():
         e0.record()
         for a, b in evs:
             a.record()
-            fn()
+            out = fn()
             b.record()
         if world > 1 and latent_model:
             eng.gather_wait()                            # the last batch's gather is inside the timed region
@@ -398,15 +426,19 @@ def main():
         t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)      # max over ranks
-        return float(t.item()), per, eng.launch_count - l0
+        return float(t.item()), per, eng.launch_count - l0, out
 
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
-    total_ms, per, launches = timed(step_device, args.steps, args.warmup)
+    total_ms, per, launches, last = timed(step_device, args.steps, args.warmup)
     clk = clocks.stop() if rank == 0 else None
     _log(f"device-resident: {total_ms / args.steps:.1f} ms/step")
-    e2e_ms, _, _ = timed(step_e2e, args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        # every path returns batch-first except raw-motion diffusion on one GPU ([T, B, 263])
+        dump_output(args.dump_outputs, OUTPUT_NAME[name], last, 1 if not latent_model and world == 1 else 0)
+    del last
+    e2e_ms, _, _, _ = timed(step_e2e, args.steps, 1)
     _log(f"e2e: {e2e_ms / args.steps:.1f} ms/step")
 
     value = world * B * args.steps / (total_ms / 1e3)
